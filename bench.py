@@ -7,6 +7,7 @@
     python bench.py --model texture --perceptual             # BASELINE configs[2] (default texture losses incl. VGG16)
     python bench.py --model joint --perceptual               # configs[4]: one warp + one texture step, 8 images/GPU
     python bench.py --device-augment                         # e2e leg with the dataset's augmentation on the device (f4)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write what the last timed step computed, DIR/*.npy
 
 One "step" = one `optimize_parameters()` of the plugin (G fwd, D step on fake+real, G step through D, both AdamW updates —
 the full reference training step, models/warp_model.py:169-183 / texture_model.py:127-180) on a synthetic batch of
@@ -30,9 +31,16 @@ libraries print (NCCL banner ...) is routed to stderr.  Field notes:
             steps (N = 1 only; --no-cpu-baseline skips it);
   --impl reference   the same port as the reference arm: exactly K timed and W warm-up steps, each on `--cpu-batch`
             image(s) of the batch (a bounded sample: the step is per-sample work + batch-mean losses), same `config`.
-            The reference is pure Python: there is nothing to compile into oracle/_ref and /root/reference does not exist
-            on the GPU box, so `kind` is "port" there; where /root/reference exists (the build container) the warp arm
-            times the UNMODIFIED reference WarpModel through its own API instead (`kind` "reference").
+            The reference is pure Python: there is nothing to compile into oracle/_ref, so `kind` is "port"; where
+            SWAPNET_REFERENCE names a checkout of the reference the warp arm times the UNMODIFIED reference WarpModel
+            through its own API instead (`kind` "reference").
+  --dump-outputs DIR  after the timed steps, what the last of them returned to its caller, one float array per file:
+            <stage>_loss_<name>.npy (float64 scalars of get_current_losses()) and <stage>_fakes.npy (float32, the
+            generator's output; above DUMP_ELEMENTS elements a fixed seeded sample of its flattened elements, the same
+            positions on every run).  Inputs and weights are seeded, so two builds can be compared file by file —
+            with a tolerance: the kernels accumulate with float atomics, and AdamW amplifies the rounding differences
+            from step to step (two runs of one build, warp, 13 steps at 512x512 batch 16 on a B200 at 1000 W: losses
+            within 1e-5 relative, fakes within 5e-2).
 """
 from __future__ import annotations
 
@@ -45,12 +53,14 @@ import tempfile
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 FULL_STEP_GFLOP_PER_IMG_512 = 1029.0   # SURVEY §8(d): full reference warp training step, nominal
+DUMP_ELEMENTS = 1 << 22                # per dumped array: 16 MB of float32, so a joint run stays under 64 MB in all
 
 
 def step_gflop_per_img(args) -> float:
@@ -207,6 +217,18 @@ def ncu_traffic():
     return None
 
 
+def dump_outputs(models, out_dir) -> None:
+    """--dump-outputs: the losses and generator output of each model's most recent step (see the module docstring)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for m in models:
+        for name, v in m.get_current_losses().items():
+            np.save(os.path.join(out_dir, f"{m.opt.model}_loss_{name}.npy"), np.float64(v))
+        fakes = m.fakes.detach().float().contiguous().cpu().numpy().ravel()
+        if fakes.size > DUMP_ELEMENTS:
+            fakes = fakes[np.unique(np.random.default_rng(0).integers(0, fakes.size, DUMP_ELEMENTS))]
+        np.save(os.path.join(out_dir, f"{m.opt.model}_fakes.npy"), fakes)
+
+
 def measured_peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -245,10 +267,10 @@ def host_cores() -> int:
 
 
 def cpu_unmodified_reference_run(S, B, steps, warmup):
-    """The UNMODIFIED reference `WarpModel` (models/warp_model.py, imported from /root/reference through
-    oracle/ref_harness.py) timed through its own public API — set_input / optimize_parameters / get_current_losses, the
-    calls of train.py:62-74 — on the host cores.  Only where /root/reference exists (the build container); the GPU
-    box has no reference tree and takes the port (`cpu_reference_run`).  -> (images/s, median s) or None."""
+    """The UNMODIFIED reference `WarpModel` (models/warp_model.py, imported from the checkout SWAPNET_REFERENCE names
+    through oracle/ref_harness.py) timed through its own public API — set_input / optimize_parameters / get_current_losses, the
+    calls of train.py:62-74 — on the host cores.  Without that checkout the arm takes the port
+    (`cpu_reference_run`).  -> (images/s, median s) or None."""
     from oracle import ref_harness as RH
 
     if not RH.available() or os.environ.get("SN_BENCH_PORT") == "1":     # SN_BENCH_PORT=1: time the port (A/B)
@@ -420,7 +442,11 @@ def main():
     ap.add_argument("--model", default="warp", choices=("warp", "texture", "joint"),
                     help="warp = the BASELINE.json metric (default); texture = configs[2]; joint = configs[4] "
                          "(one warp step + one texture step per iteration)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the losses and the generator output of the last one as DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the timed CUDA path computed: --impl b200 only")
     _protect_stdout()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -466,8 +492,7 @@ def main():
                              "sample": f"{args.steps} timed + {args.warmup} warm-up full training steps at {S}x{S}, each on "
                                        f"{args.cpu_batch} image(s) of the batch (bounded sample), torch CPU fp32 "
                                        f"({cores} threads = usable host cores); oracle/nets.py, pinned bit-exactly to the "
-                                       "reference modules (the reference is pure Python: nothing to compile into oracle/_ref, "
-                                       "and /root/reference does not exist on the GPU box)"},
+                                       "reference modules (the reference is pure Python: nothing to compile into oracle/_ref)"},
             "e2e": {"value": v, "unit": "images/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}))
         return
 
@@ -552,6 +577,8 @@ def main():
     ms = timed(args.steps, False, False)
     launches = ops.launch_count() - l0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:     # before the e2e leg's steps move the weights on
+        dump_outputs([m for m, *_ in legs], args.dump_outputs)
     for _ in range(2):                      # the host-input path has its own staging buffers: warm them
         one_step(True, True)
     ms_e2e = timed(args.steps, True, True)

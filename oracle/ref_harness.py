@@ -1,6 +1,6 @@
-"""TEST INFRASTRUCTURE ONLY — imports the UNMODIFIED reference from /root/reference (build container
-only; the GPU box has no /root/reference) so that the oracle restatement can be pinned against it and
-golden vectors generated (tests/tools/make_golden.py).  Recipe: SURVEY.md App. C.
+"""TEST INFRASTRUCTURE ONLY — imports the UNMODIFIED reference from a checkout of andrewjong/SwapNet named by the
+environment variable SWAPNET_REFERENCE, so that the golden vectors under tests/golden/ can be generated from it
+(tests/tools/make_golden*.py).  Recipe: SURVEY.md App. C.
 """
 from __future__ import annotations
 
@@ -12,11 +12,11 @@ import types
 
 import torch
 
-REF = "/root/reference"
+REF = os.path.abspath(os.environ["SWAPNET_REFERENCE"]) if os.environ.get("SWAPNET_REFERENCE") else None
 
 
 def available() -> bool:
-    return os.path.isdir(os.path.join(REF, "models"))
+    return REF is not None and os.path.isdir(os.path.join(REF, "models"))
 
 
 def _install_stubs() -> None:
@@ -36,7 +36,7 @@ def _install_stubs() -> None:
 
 def import_reference():
     """Put the reference first on sys.path (its packages are called models/modules/...)."""
-    assert available(), "reference tree not mounted"
+    assert available(), "set SWAPNET_REFERENCE to a checkout of the reference"
     _install_stubs()
     if REF not in sys.path:
         sys.path.insert(0, REF)

@@ -1,8 +1,8 @@
 """CPU tests of the device-side input pipeline's host half and of its oracle (SURVEY §8 f4).
 
   * oracle/augment.py (numpy restatement of Pillow's resampling) is pinned bit-exactly against Pillow / torchvision
-    themselves, against the reference's own `per_channel_transform(get_transforms(opt))` when /root/reference is
-    importable, and against tests/golden/augment_64.npz (generated from the reference);
+    themselves and against what the reference's own `per_channel_transform(get_transforms(opt))` produced
+    (tests/golden/augment_64.npz, tests/golden/reference_datasets.npz);
   * swapnet_b200.data.draw_channel_ops makes the reference's random draws without touching pixels: same ops, and the
     python `random` / torch generators end in the same state.
 The device kernel is compared with the same oracle in tests/test_augment_gpu.py.
@@ -20,16 +20,16 @@ from torchvision import transforms as T
 from torchvision.transforms import functional as TF
 
 from oracle import augment as A
-from oracle import ref_harness as RH
 from swapnet_b200 import data as D
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "augment_64.npz")
+REFERENCE_DATASETS = os.path.join(os.path.dirname(__file__), "golden", "reference_datasets.npz")
 SIZES = [(64, 64), (128, 96), (37, 53), (512, 512)]
 
 
 def reference_transform(names):
-    """datasets/__init__.py:88-110 `get_transforms` restated with the same torchvision objects (the GPU box has no
-    /root/reference); `test_matches_the_reference_function` checks the real one."""
+    """datasets/__init__.py:88-110 `get_transforms` restated with the same torchvision objects;
+    `test_matches_the_reference_function` checks it against the real one."""
     tl = []
     every = "all" in names
     if every or "vflip" in names:
@@ -116,23 +116,19 @@ def test_host_draws_plus_oracle_equal_the_pillow_pipeline(names, size):
         assert np.array_equal(A.per_channel_transform(planes, ops), ref)
 
 
-@pytest.mark.skipif(not RH.available(), reason="needs /root/reference (build container)")
 def test_matches_the_reference_function():
-    RH.import_reference()
-    from datasets import get_transforms
-    from datasets.data_utils import per_channel_transform
-
-    tf = get_transforms(Namespace(input_transforms=("hflip", "vflip", "affine", "perspective")))
-    lab = label_map(96, 96, 7)
-    cloth = torch.from_numpy(A.onehot(lab, 19))
+    """The reference's own `get_transforms` + `per_channel_transform` on a 96x96 label map, stored by
+    tests/tools/make_golden_reference.py: `reference_transform` builds the same transform object, and the host draws +
+    oracle give the same pixels and leave both generators in the same state."""
+    z = np.load(REFERENCE_DATASETS)
+    tf = reference_transform(tuple(str(z["transforms"]).split(",")))
+    assert repr(tf) == str(z["transforms_repr"])
+    cloth = A.onehot(label_map(96, 96, 7), 19)
     for seed in (0, 1, 2):
         random.seed(seed); torch.manual_seed(seed)
-        ref = per_channel_transform(cloth, tf).numpy()
-        state = rng_digest()
-        random.seed(seed); torch.manual_seed(seed)
         ops = D.draw_channel_ops(tf, 19, 96, 96)
-        assert rng_digest() == state
-        assert np.array_equal(A.per_channel_transform(cloth.numpy(), ops), ref)
+        assert rng_digest() == str(z[f"seed{seed}_rng"])
+        assert np.array_equal(A.per_channel_transform(cloth, ops), z[f"seed{seed}_out"])
 
 
 def test_golden_fixture_from_the_reference():
@@ -175,11 +171,8 @@ def test_load_label_map_equals_the_reference_decompression(tmp_path):
     sparse.save_npz(fname, sparse.csc_matrix(lab.astype(np.int64)))      # data_utils.py:311-327 compress_and_save_cloth
     got = D.load_label_map(fname)
     assert got.dtype == np.uint8 and np.array_equal(got, lab)
-    if RH.available():
-        RH.import_reference()
-        from datasets.data_utils import decompress_cloth_segment
-
-        assert np.array_equal(A.onehot(got, 19), decompress_cloth_segment(fname, 19).numpy())
+    # the reference's decompress_cloth_segment(fname, 19) of the same file (tests/tools/make_golden_reference.py)
+    assert np.array_equal(A.onehot(got, 19), np.load(REFERENCE_DATASETS)["decompressed_48x40"])
 
 
 def test_kernel_source_run_on_the_host_equals_oracle(tmp_path):

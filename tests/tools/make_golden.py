@@ -1,6 +1,6 @@
-"""Generate tests/golden/*.pt from the UNMODIFIED reference (/root/reference) — build container only.
+"""Generate tests/golden/*.pt from the UNMODIFIED reference (oracle/ref_harness.py).
 
-    python tests/tools/make_golden.py
+    SWAPNET_REFERENCE=/path/to/SwapNet python tests/tools/make_golden.py
 
 Fixtures (all seeded; see tests/test_oracle_cpu.py for how they are consumed):
   warp_64.pt     reference WarpModule / define_D forward (eval) + one full reference

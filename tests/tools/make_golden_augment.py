@@ -1,6 +1,6 @@
-"""Generate tests/golden/augment_64.npz from the UNMODIFIED reference (/root/reference) — build container only.
+"""Generate tests/golden/augment_64.npz from the UNMODIFIED reference (oracle/ref_harness.py).
 
-    python tests/tools/make_golden_augment.py
+    SWAPNET_REFERENCE=/path/to/SwapNet python tests/tools/make_golden_augment.py
 
 The reference's own `per_channel_transform` (datasets/data_utils.py:346-361) with its own `get_transforms(opt)`
 (datasets/__init__.py:88-110; warp default --input_transforms hflip vflip affine perspective) on a seeded 19-channel

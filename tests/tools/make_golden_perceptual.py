@@ -1,7 +1,7 @@
 """Generate tests/golden/perceptual_64.pt from the UNMODIFIED reference PerceptualLoss
-(/root/reference/modules/losses/perceptual.py) — build container only.
+(modules/losses/perceptual.py of the checkout oracle/ref_harness.py imports).
 
-    python tests/tools/make_golden_perceptual.py
+    SWAPNET_REFERENCE=/path/to/SwapNet python tests/tools/make_golden_perceptual.py
 
 `vgg16(pretrained=True)` (perceptual.py:26) is a download and impossible offline: the constructor is patched
 to torchvision's own seeded random init (torch.manual_seed(1234)), the same stand-in the B200 plugin uses with

@@ -1,8 +1,8 @@
 """Generate tests/golden/texture_step_64.pt: ONE full reference `TextureModel.optimize_parameters()`
-(/root/reference/models/texture_model.py:127-180, base_gan.py:194-203) with the reference's DEFAULT losses
-(L1 10, GAN 1, VGG16 content 20, Gram style 1e-8) — build container only.
+(models/texture_model.py:127-180, base_gan.py:194-203) with the reference's DEFAULT losses
+(L1 10, GAN 1, VGG16 content 20, Gram style 1e-8), imported through oracle/ref_harness.py.
 
-    python tests/tools/make_golden_texture_step.py
+    SWAPNET_REFERENCE=/path/to/SwapNet python tests/tools/make_golden_texture_step.py
 
 CPU (gpu_id=None), eval-mode nets (torch's dropout RNG cannot be restated), 64x64, batch 2.  `vgg16(pretrained=True)`
 (modules/losses/perceptual.py:26) is patched to torchvision's seeded random init (see make_golden_perceptual.py).
